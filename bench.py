@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- surfel-rasterizer forward+backward frames/s at 512x512 / 300 K surfels (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -25,10 +25,18 @@ One JSON line (rank 0):
 
 --impl reference runs the UNMODIFIED reference extension (oracle/_ref/_C.so, its own CUDA path) through the same
 harness; if the .so is missing it falls back to the CPU oracle port and says so.
+
+--dump-outputs DIR writes what the last timed step of the value arm computed (rank 0), as float32 .npy files a caller
+of that path would receive: color (F,3,n) and allmap (F,8,n) at n pixels, radii (F,m), and the frame-summed surfel
+gradients dL_dmeans3D / dL_dsh / dL_dopacity / dL_dscales / dL_drotations (m,...) of m surfels.  n and m are every
+pixel and surfel when the files fit in 64 MB, otherwise a fixed sample of them: sorted indices drawn by
+np.random.default_rng(0) (pixels) and np.random.default_rng(1) (surfels).  The inputs are seeded, so two builds run
+with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import contextlib
 import json
 import os
@@ -50,12 +58,14 @@ from vidu4d_b200.synthetic import SurfelCloud, object_scene, orbit_view, project
 NVIEWS = 64
 TAN = 0.5
 L2_MB = 126
+GRAD_KEYS = ("dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations")      # the flat gradient buffer, in order
+DUMP_BYTES = 63 * 10**6     # --dump-outputs: array bytes, leaving room for the .npy headers under 64 MB
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--surfels", type=int, default=300_000)
@@ -76,7 +86,11 @@ def parse():
     ap.add_argument("--no-fused", action="store_true", help="e2e through render() instead of render_fused()")
     ap.add_argument("--e2e-streams", type=int, default=1, help="(debug) streams of the eager e2e step when --no-graph")
     ap.add_argument("--streams", type=int, default=8, help="CUDA streams the frames of a step alternate over (value arm)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed value-arm step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -93,6 +107,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "100", "-i", str(self.index)], stdout=subprocess.PIPE,
                                          stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)         # never outlive the benchmark, even when it fails before stop()
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -164,6 +179,8 @@ def main():
     args = parse()
     rank, world, local_rank = D.env_rank_world()
     if args.impl == "reference" and (args.ref_device == "cpu" or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "_C.so"))):
+        if args.dump_outputs:
+            sys.exit("--dump-outputs: the CPU oracle arm has no GPU outputs to write")
         return reference_cpu_arm(args, rank, world)
     assert torch.cuda.is_available(), "bench.py needs a GPU (the CPU oracle is only the baseline leg)"
     device = torch.device("cuda", local_rank)
@@ -245,11 +262,11 @@ def main():
         return out
     accs = [views(stack[k]) for k in range(NS)]
     flat_views = views(flat_acc)
-    flat_outs = dict(zip(("dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"), flat_views))
+    flat_outs = dict(zip(GRAD_KEYS, flat_views))
     # second flat gradient buffer: the two captured value-arm steps each write their own, so that step k's all-reduce can
     # run on the communication stream while step k+1 computes (multi-GPU only; see step_dev)
     flat_acc2 = torch.zeros((nflt,), device=device) if (BATCH and world > 1) else flat_acc
-    flat_outs2 = dict(zip(("dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"), views(flat_acc2)))
+    flat_outs2 = dict(zip(GRAD_KEYS, views(flat_acc2)))
     flat_accs, flat_outss = [flat_acc, flat_acc2], [flat_outs, flat_outs2]
     GIDX = (3, 5, 2, 6, 7)      # gr = (dmeans2D, dcolors, dopacity, dmeans3D, dtransMat, dsh, dscales, drots)
     step_ctr = torch.zeros((), dtype=torch.int64, device=device)      # lives on the device: the captured step advances it
@@ -261,12 +278,12 @@ def main():
 
     SPLIT = max(1, args.split) if BATCH else 1
     split_rows = torch.zeros((SPLIT, nflt), device=device) if SPLIT > 1 else None
-    split_outs = [dict(zip(("dL_dmeans3D", "dL_dsh", "dL_dopacity", "dL_dscales", "dL_drotations"), views(split_rows[k])))
+    split_outs = [dict(zip(GRAD_KEYS, views(split_rows[k])))
                   for k in range(SPLIT)] if SPLIT > 1 else None
 
     def batch_body(fpc=None, slot=0):
         """One batched forward+backward of `fpc` frames (default F) + the sum over frames into the flat gradient
-        (buffer `slot`)."""
+        (buffer `slot`).  Returns the forward outputs of each launch and the flat gradient buffer written."""
         n = F if fpc is None else fpc
         idx = (step_ctr * (world * F) + rank * F + ar[:n]) % NVIEWS
         step_ctr.add_(1)
@@ -274,20 +291,21 @@ def main():
         if SPLIT > 1 and n == F:
             main = torch.cuda.current_stream()
             sub = F // SPLIT
-            o = None
+            fwd = []
             for k in range(SPLIT):
                 side[k].wait_stream(main)
                 with torch.cuda.stream(side[k]):
                     sl = slice(k * sub, (k + 1) * sub)
                     o = C.rasterize_gaussians_batch(bg, t_in["means3D"], e, t_in["opac"], t_in["scales"], t_in["rots"], 1.0, vm_b[sl],
                                                     pm_b[sl], TAN, TAN, RES, RES, t_in["shs"], 3, cp_b[sl])
+                    fwd.append(o)
                     C.rasterize_gaussians_backward_batch(bg, t_in["means3D"], o[3], e, t_in["scales"], t_in["rots"], 1.0, vm_b[sl],
                                                          pm_b[sl], TAN, TAN, dLc_b[sl], dLo_b[sl], t_in["shs"], 3, cp_b[sl], o[4], o[5],
                                                          o[6], sum_shared=True, want_transmat=False, outs=split_outs[k])
             for k in range(SPLIT):
                 main.wait_stream(side[k])
             torch.sum(split_rows, dim=0, out=flat_acc)
-            return o
+            return fwd, flat_acc
         o = C.rasterize_gaussians_batch(bg, t_in["means3D"], e, t_in["opac"], t_in["scales"], t_in["rots"], 1.0, vm_b, pm_b,
                                         TAN, TAN, RES, RES, t_in["shs"], 3, cp_b)
         # gradients of the (shared) surfel parameters are summed over the frames inside the per-surfel kernel and land
@@ -298,7 +316,8 @@ def main():
         if n != F:      # the 1- and 2-frames-per-call variants: several calls per step accumulate into the flat buffer
             for a_, gi in zip(flat_views, GIDX):
                 a_.add_(gr[gi].reshape(a_.shape))
-        return o
+            return [o], flat_acc
+        return [o], flat_accs[slot]
 
     # Two captures of the same step, used alternately, each with its own pinned status words and a "done" event: the host
     # checks step k-1's overflow words only AFTER it has queued step k, so the GPU never waits for the host between steps
@@ -325,12 +344,15 @@ def main():
             if ar_pending[k]:
                 torch.cuda.current_stream().wait_event(ar_done[k]); ar_pending[k] = False
 
+    last_out = [None]       # (forward outputs, flat gradient buffer) of the latest step, for --dump-outputs
+
     def step_dev(step):
         R_last = 0
         if BATCH:
             if value_graph[0] is not None:
                 k = step & 1
                 value_graphs[k].replay()
+                last_out[0] = value_graphs[k].result
                 if world > 1:
                     # step k's all-reduce (its own flat buffer) goes to the communication stream and overlaps step k+1's
                     # compute; this step's timed interval ends only after the PREVIOUS step's all-reduce has finished, so
@@ -347,7 +369,7 @@ def main():
                 drain()                     # step k-1 (the other graph): its words landed long ago
                 inflight[0] = k
                 return R_last
-            batch_body()
+            last_out[0] = batch_body()
             if world > 1:
                 torch.distributed.all_reduce(flat_acc)
             RZ.check_overflow()             # eager fallback: the step's only host<->device synchronisation
@@ -356,6 +378,7 @@ def main():
         if NS > 1:
             for st_ in side:
                 st_.wait_stream(main)
+        fwd = []
         for f in range(F):
             k = f % NS
             ctx = torch.cuda.stream(side[k]) if NS > 1 else contextlib.nullcontext()
@@ -367,6 +390,9 @@ def main():
                     else:
                         a_.add_(gr[gi].view(a_.shape))
                 R_last = o[0]
+                if args.dump_outputs:
+                    fwd.append(o[:4])
+        last_out[0] = (fwd, flat_acc)
         if NS > 1:
             for st_ in side:
                 main.wait_stream(st_)
@@ -398,7 +424,7 @@ def main():
             gph = torch.cuda.CUDAGraph()
             lc0 = _capi.launch_count()
             with torch.cuda.graph(gph):
-                body_fn()
+                gph.result = body_fn()          # the graph's outputs: every replay rewrites these tensors
             gph.launches = _capi.launch_count() - lc0      # kernels of OUR library one replay launches
             gph.watch = list(RZ._pending)      # the pinned status words this graph rewrites on every replay
             return gph
@@ -457,6 +483,8 @@ def main():
     if BATCH:
         arm(value_graph[0])
     total_ms, per_ms, wall_ms = timed(step_dev, K, Wm)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last_out[0], views)
     launches = (_capi.launch_count() - launches0) if args.impl == "ours" else None
     if BATCH and value_graph[0] is not None:
         launches = value_graph[0].launches * K          # graph replays do not pass through the library's host-side counter
@@ -889,6 +917,32 @@ def main():
     if world > 1:
         torch.distributed.destroy_process_group()
     return 0
+
+
+def dump_outputs(dirname, fwd, grad_flat, views):
+    """--dump-outputs (see the module docstring): fwd = the forward outputs (num_rendered, color, allmap, radii, ...) of
+    the step's launches in frame order, grad_flat = the flat gradient buffer the step wrote."""
+    color = torch.cat([o[1].reshape(-1, 3, o[1].shape[-2] * o[1].shape[-1]) for o in fwd])
+    allmap = torch.cat([o[2].reshape(-1, 8, o[2].shape[-2] * o[2].shape[-1]) for o in fwd])
+    radii = torch.cat([o[3].reshape(-1, o[3].shape[-1]) for o in fwd]).float()
+    grads = dict(zip(GRAD_KEYS, views(grad_flat)))
+    F, n_pix, n_surf = color.shape[0], color.shape[-1], radii.shape[-1]
+    pixel_bytes = F * (3 + 8) * 4
+    surfel_bytes = (F + sum(g[0].numel() for g in grads.values())) * 4
+    n, m = n_pix, n_surf
+    while n * pixel_bytes + m * surfel_bytes > DUMP_BYTES:
+        n, m = (n + 1) // 2, (m + 1) // 2
+    dev = color.device
+    pix = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n_pix, n, replace=False))).to(dev) if n < n_pix else None
+    surf = torch.from_numpy(np.sort(np.random.default_rng(1).choice(n_surf, m, replace=False))).to(dev) if m < n_surf else None
+    out = {"color": color, "allmap": allmap, "radii": radii, **grads}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        if name in ("color", "allmap"):
+            a = a if pix is None else a.index_select(-1, pix)
+        else:
+            a = a if surf is None else a.index_select(-1 if name == "radii" else 0, surf)
+        np.save(os.path.join(dirname, name + ".npy"), a.float().cpu().numpy())
 
 
 def cpu_oracle_fps(scene, vms_h, pms_h, cps_h, RES, nframes, dLc, dLo):
